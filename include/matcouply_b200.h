@@ -287,6 +287,22 @@ int b2_quadform(const void* M, const void* x, int n_groups, int J, int R, double
 int b2_pf2_fixed_basis(void* pd, void* dual, const void* P, const void* Delta, const int64_t* row_off, int n_groups,
                        long long n, int R, const void* rho, double* num_part, int phase, int dtype, void* stream);
 
+/* ---- masked fitting (missing entries, EM refill after every outer iteration; DESIGN.md §10) --------------------
+ * Missing-entry refill.  For every packed row n (slice g = group_of_row[n]) and every missing column k in
+ * miss_col[miss_row_ptr[n] .. miss_row_ptr[n+1]) (int64 row pointer of n_rows+1 entries, int32 columns < K):
+ *   xhat = sum_r B[n][r] A[g][r] C[k][r];   d = xhat - X[n][k]   (X[n][k] = the fill the iteration just used)
+ *   out[0] += (X[n][k] - xhat)^2      missing-entry part of ||F - X_hat||^2
+ *   out[1] += xhat^2 - X[n][k]^2      change of ||F||^2
+ *   Y[n][:] += d * C[k][:]             keeps Y = F C valid (Y may be NULL)
+ *   X[n][k]  = xhat
+ * X: n_rows x K with row stride ldx; A (I x R), B and Y (n_rows x R), C (K x R) dense.  fp32 / fp64 like the engine;
+ * sums in double, reduced in a fixed order (no atomics on the sums: runs are bit-reproducible, as everywhere else in
+ * this library).  ws: >= b2_mask_refill_workspace_bytes(n_rows) bytes. */
+int b2_mask_refill(void* X, long long n_rows, int K, int ldx, const int64_t* miss_row_ptr, const int32_t* miss_col,
+                   const int32_t* group_of_row, const void* A, const void* B, const void* C, int R, void* Y,
+                   double* out, int dtype, void* ws, size_t ws_bytes, void* stream);
+size_t b2_mask_refill_workspace_bytes(long long n_rows);
+
 /* ---- initial state: device-side continuation of a NumPy RandomState (MT19937) stream ----------------------------
  * out[0:n] = the next n doubles `np.random.RandomState.random_sample` / `uniform(0, 1)` would return for the generator
  * whose state is state_io (device, 625 uint32: the 624 key words and the position, as in RandomState.get_state());

@@ -238,6 +238,76 @@ class ShardRows:
         raise RuntimeError(f"only slices [{self.lo}, {self.hi}) of this variable exist on this rank")
 
 
+class MaskCSR:
+    """The missing entries of a mask as a CSR list over the packed rows: row n misses the columns
+    ``col[row_ptr[n]:row_ptr[n+1]]`` (ascending).  ``row_ptr`` is int64 (N + 1), ``col`` int32; NumPy arrays when
+    packed on the host, CUDA tensors once on the device."""
+
+    def __init__(self, row_ptr, col, n_observed):
+        self.row_ptr, self.col = row_ptr, col
+        self.n_missing = int(row_ptr[-1]) if len(row_ptr) else 0
+        self.n_observed = int(n_observed)
+
+    def to(self, device):
+        if isinstance(self.row_ptr, torch.Tensor):
+            return MaskCSR(self.row_ptr.to(device), self.col.to(device), self.n_observed)
+        return MaskCSR(torch.as_tensor(self.row_ptr).to(device), torch.as_tensor(self.col).to(device),
+                       self.n_observed)
+
+    def flat_index(self, ldx):
+        """int64 offsets ``row * ldx + col`` of the missing entries in the flattened packed data (device tensors)."""
+        n_rows = self.row_ptr.numel() - 1
+        rows = torch.repeat_interleave(torch.arange(n_rows, device=self.col.device), torch.diff(self.row_ptr))
+        return rows * int(ldx) + self.col.to(torch.int64)
+
+
+def pack_mask(mask, shapes, require_observed=True):
+    """Host packing of a per-slice mask (list of ``J_i x K`` arrays, NumPy or torch, bool or 0/1; 1 = observed) for
+    data of the given slice shapes.  Raises ValueError for a shape mismatch, entries other than 0/1 or a mask without
+    any observed entry."""
+    shapes = [tuple(int(d) for d in s) for s in shapes]
+    mask = list(mask)
+    if len(mask) != len(shapes):
+        raise ValueError(f"mask has {len(mask)} slices, the data has {len(shapes)}")
+    counts, cols, n_obs = [np.zeros(1, dtype=np.int64)], [], 0
+    for i, (m, s) in enumerate(zip(mask, shapes)):
+        if isinstance(m, torch.Tensor):
+            m = m.detach().cpu().numpy()
+        m = np.asarray(m)
+        if m.shape != s:
+            raise ValueError(f"mask slice {i} has shape {m.shape}, the data slice has shape {s}")
+        if m.dtype != np.bool_:
+            if not np.all((m == 0) | (m == 1)):
+                raise ValueError(f"mask slice {i} has entries other than 0 and 1")
+            m = m != 0
+        missing = ~m.reshape(s)
+        counts.append(missing.sum(axis=1, dtype=np.int64))
+        flat = np.flatnonzero(missing)  # row-major: ascending columns within each row
+        cols.append((flat % max(s[1], 1)).astype(np.int32))
+        n_obs += int(m.sum())
+    if n_obs == 0 and require_observed:
+        raise ValueError("the mask has no observed entry")
+    row_ptr = np.cumsum(np.concatenate(counts)).astype(np.int64)
+    col = np.concatenate(cols) if cols else np.zeros(0, dtype=np.int32)
+    return MaskCSR(row_ptr, col, n_obs)
+
+
+def pack_mask_device(mask, packed, require_observed=True):
+    """Device packing of one ``(N, K)`` bool CUDA tensor over the packed rows of `packed` (PackedMatrices)."""
+    if not isinstance(mask, torch.Tensor) or mask.dtype != torch.bool or mask.device != packed.X.device:
+        raise ValueError(f"a single-tensor mask must be a bool tensor on {packed.X.device}")
+    if tuple(mask.shape) != (packed.N, packed.K):
+        raise ValueError(f"mask has shape {tuple(mask.shape)}, the packed data is {(packed.N, packed.K)}")
+    missing = ~mask
+    n_obs = int(mask.sum())
+    if n_obs == 0 and require_observed:
+        raise ValueError("the mask has no observed entry")
+    row_ptr = torch.zeros(packed.N + 1, dtype=torch.int64, device=mask.device)
+    torch.cumsum(missing.sum(dim=1), 0, out=row_ptr[1:])
+    col = torch.nonzero(missing)[:, 1].to(torch.int32)  # row-major order: ascending within each row
+    return MaskCSR(row_ptr, col, n_obs)
+
+
 class _ModeState:
     """Factor matrix + per-penalty aux/dual of one mode, all flat (n x R) device tensors."""
 
@@ -253,7 +323,7 @@ class _ModeState:
 class AOADMMEngine:
     def __init__(self, packed, rank, regs, l2_penalty=(0, 0, 0), feasibility_penalty_scale=1.0, constant_A=False,
                  constant_B=False, inner_n_iter_max=5, update=(True, True, True), group=None, xstream_variant=None,
-                 fuse_local=None, fuse_pf2=None, shard_rows=None, inner_tol=None, fuse_x1=None):
+                 fuse_local=None, fuse_pf2=None, shard_rows=None, inner_tol=None, fuse_x1=None, mask=None):
         _lib.load()
         self.p = packed
         self.dev = packed.X.device
@@ -382,6 +452,16 @@ class AOADMMEngine:
             self.fws = _ops.FusedWorkspace(packed.row_offsets, K, R, dev)
         self.scal = torch.zeros(64, dtype=torch.float64, device=dev)
         self.normX_sq = None
+        # Masked fitting (MaskCSR of the missing entries, or None): X holds the filled data F, whose missing entries are
+        # refilled from the model after every outer iteration.  msum = [missing-entry part of ||F - X_hat||^2 of the
+        # last refill, ||F||^2, ||F||^2 before the last refill]; kept out of `scal`, which is cleared per evaluation.
+        self.mask = None
+        if mask is not None:
+            self.mask = mask.to(dev)
+            if self.mask.row_ptr.numel() != N + 1:
+                raise ValueError(f"the mask covers {self.mask.row_ptr.numel() - 1} rows, the data has {N}")
+            self.msum = torch.zeros(3, dtype=torch.float64, device=dev)
+            self.mask_ws = _ops.mask_refill_workspace(N, dev)
         uni = None
         if any(d[0] == _lib.PEN_UNIMODAL for d in self.modes[1].desc):
             uni = (I, R, self.max_rows)
@@ -958,13 +1038,33 @@ class AOADMMEngine:
         return full
 
     def prepare(self):
-        """Before the first iteration: ||X||^2 and the products for the initial fit (decomposition.py:906-913)."""
+        """Before the first iteration: ||X||^2 and the products for the initial fit (decomposition.py:906-913).
+        With a mask: the missing entries are zeroed, so that ||X||^2 = ||M o X||^2, and then filled from the initial
+        factors (F^(0))."""
         out = self.scal[60:61]
+        if self.mask is not None:
+            self.p.X.view(-1)[self.mask.flat_index(self.p.X.shape[1])] = 0
         _ops.sumsq(self.p.X, self.N, self.K, out, self.ws)
+        if self.mask is not None:
+            self.msum[1].copy_(out[0])  # rank-local ||F||^2
         self._allreduce(out)
         self.normX_sq = float(out.item())
         _ops.slice_gram(self.modes[1].x, self.row_off, self.I, self.R, self.BtB)
+        if self.mask is not None:
+            self.refill(None)
+            # F^(0) equals the initial model at the missing entries: the initial fit has no missing-entry term
+            self.msum[2].copy_(self.msum[1])
+            self.msum[0].zero_()
         self.refresh_products()
+
+    def refill(self, Y):
+        """F <- M o X + (1 - M) o X_hat(A, B, C) (b2_mask_refill); Y += the matching rank-R correction (if given)."""
+        m = self.mask
+        self.msum[2].copy_(self.msum[1])
+        self.msum[0].zero_()
+        self._timed("refill", lambda: _ops.mask_refill(
+            self.p.X, self.N, self.K, m.row_ptr, m.col, self.gor, self.modes[0].x, self.modes[1].x, self.modes[2].x, Y,
+            self.msum[0:2], self.mask_ws))
 
     def outer_iteration(self):
         """One pass of decomposition.py:945-988."""
@@ -974,12 +1074,17 @@ class AOADMMEngine:
         if self.update_C:
             with _Phase("b2:admm_update_C"):
                 self.step_C()
-        if self.update_B or self.update_C:
+        if self.update_B or self.update_C or self.mask is not None:  # F, and with it X C, changes with every refill
             with _Phase("b2:xstream_y+products"):
                 self.refresh_products()
         if self.update_A:
             with _Phase("b2:admm_update_A"):
                 self.step_A()
+        if self.mask is not None:
+            with _Phase("b2:mask_refill"):
+                # the next B-update reads the cached Y = F C (two-pass schedule, PARAFAC2 row pass) unless it is the
+                # single-read fused pass, which computes its own Y from X
+                self.refill(None if self.fused_x1 else self.Y)
 
     # ------------------------------------------------------------------------------------------------------
     # diagnostics: one fused scalar pack, one device->host copy
@@ -1000,6 +1105,10 @@ class AOADMMEngine:
         scal.zero_()
         slot = 2  # [0:2] fit terms
         _ops.fit_terms(self.rhsA, self.cross, self.modes[0].x, self.I, self.R, scal[0:2], self.ws)
+        if self.mask is not None:  # [2:4] ||F^(t-1)||^2 and the missing-entry term (rank-local: all-reduced part)
+            scal[2].copy_(self.msum[2])
+            scal[3].copy_(self.msum[0])
+            slot = 4
         layout, deferred_A = [], []
         sizes = (self.I * self.R, self.N * self.R, self.K * self.R)
         # sharded modes first (A, B), replicated mode (C) last
@@ -1060,7 +1169,10 @@ class AOADMMEngine:
             if p >= 0:
                 gaps[m].append(np.sqrt(d2) / np.sqrt(x2))
                 l1[m].append(ab)
-        return dict(gaps=gaps, fit=(host[0], host[1]), sq=sq, l1=l1, extra=extra)
+        out = dict(gaps=gaps, fit=(host[0], host[1]), sq=sq, l1=l1, extra=extra)
+        if self.mask is not None:
+            out["masked"] = (host[2], host[3])
+        return out
 
     # ------------------------------------------------------------------------------------------------------
     # CUDA-graph replay of the steady-state outer iteration (launch-bound problem sizes)

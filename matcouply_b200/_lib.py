@@ -79,6 +79,7 @@ _SIGNATURES = {
     "b2_mt19937_uniform": [_vp, _vp, _ll, _vp],
     "b2_mt19937_jump_host": [_vp, ctypes.c_ulonglong],
     "b2_set_option": [_i, _i],
+    "b2_mask_refill": [_vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _vp, _sz, _vp],
 }
 _OTHER = {
     "b2_last_error": ([], ctypes.c_char_p),
@@ -92,6 +93,7 @@ _OTHER = {
     "b2_xstream_fused_workspace_bytes": ([_i, _i, _i], _sz),
     "b2_xstream_z_ldw": ([_i, _i, _i], _i),
     "b2_unimodal_workspace_bytes": ([_i, _i, _i], _sz),
+    "b2_mask_refill_workspace_bytes": ([_ll], _sz),
 }
 EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + list(_OTHER))
 

@@ -144,6 +144,17 @@ def sumsq(X, n_rows, K, out, ws):
          _stream())
 
 
+def mask_refill_workspace(n_rows, device):
+    """Scratch of b2_mask_refill for n_rows packed rows."""
+    return torch.empty(int(_lib.load().b2_mask_refill_workspace_bytes(int(n_rows))), dtype=torch.uint8, device=device)
+
+
+def mask_refill(X, n_rows, K, row_ptr, miss_col, gor, A, B, C, Y, out, ws):
+    """Missing entries of X <- (B o A[gor]) C^T, Y += d C (Y may be None), out[0:2] += (sum d^2, change of ||X||^2)."""
+    call("b2_mask_refill", _ptr(X), n_rows, K, X.shape[1], _ptr(row_ptr), _ptr(miss_col), _ptr(gor), _ptr(A), _ptr(B),
+         _ptr(C), C.shape[1], _ptr(Y), _ptr(out), dtype_code(X.dtype), _ptr(ws), ws.numel(), _stream())
+
+
 def gram(M, n, G, ws):
     call("b2_gram", _ptr(M), n, G.shape[0], M.shape[1], _ptr(G), dtype_code(M.dtype), _ptr(ws.red), ws.red_bytes,
          _stream())

@@ -297,9 +297,15 @@ def compute_feasibility_gaps(cmf, regs, A_aux_list, B_aux_list, C_aux_list):
 
 
 def _loss(diag, norm_X_sq, l2_penalty, regs, host_factors=None):
-    """0.5*rel_err^2 + 0.5*sum_m lambda_m ||factor_m||^2 + sum penalties (decomposition.py:1013-1023)."""
+    """0.5*rel_err^2 + 0.5*sum_m lambda_m ||factor_m||^2 + sum penalties (decomposition.py:1013-1023).  With a mask,
+    ``norm_X_sq`` is ||M o X||^2 and the error is the one over the observed entries: ||F - X_hat||^2 of the filled data
+    F the iteration ran on, less its missing-entry part."""
     inner, quad = diag["fit"]
-    rec_error = np.sqrt(max(0, norm_X_sq - 2 * inner + quad)) / np.sqrt(norm_X_sq)
+    if "masked" in diag:
+        norm_F_sq, missing_sq = diag["masked"]
+        rec_error = np.sqrt(max(0, norm_F_sq - 2 * inner + quad - missing_sq)) / np.sqrt(norm_X_sq)
+    else:
+        rec_error = np.sqrt(max(0, norm_X_sq - 2 * inner + quad)) / np.sqrt(norm_X_sq)
     l2reg = 0
     for m in range(3):
         if l2_penalty[m]:
@@ -440,6 +446,7 @@ def cmf_aoadmm(
     shard=None,
     gather_factors=True,
     use_cuda_graph=None,
+    mask=None,
 ):
     """Fit a regularized coupled matrix factorization with AO-ADMM on a B200 (same signature and semantics as the
     reference ``matcouply.decomposition.cmf_aoadmm``, decomposition.py:662-1100).
@@ -456,12 +463,33 @@ def cmf_aoadmm(
     ``n_iter_max >= 16`` (config 1: 2.01 -> 1.91 ms per iteration; with PARAFAC2 the replay does not pay — README
     configuration 0.76 ms eager and replayed alike, config 3 slower); ``True`` = wherever the engine allows it
     (single GPU, data <= 1 GB or no PARAFAC2); ``False`` = never.  Same kernels on the same buffers: bit-identical.
+
+    ``mask``: fit data with missing entries (1 / True = observed, 0 / False = missing), as a list of per-slice arrays
+    shaped like ``matrices`` (NumPy or torch, bool or 0/1) or, for :class:`matcouply_b200.PackedMatrices` input, also
+    one ``(N, K)`` bool CUDA tensor on the data's device; with ``shard`` it holds this rank's slices, as ``matrices``
+    does.  The fit is EM-style with one refill per outer iteration.  The iteration runs on filled data
+    ``F = M o X + (1 - M) o X_hat``, built first from the initial factors (``X`` is never read at missing positions:
+    NaN or inf there is fine).  Every outer iteration runs the unchanged B-, C- and A-updates on ``F`` and then refills
+    the missing entries from the new factors.  ``rec_errors`` is the relative error over the observed entries,
+    ``||M o (X - X_hat)|| / ||M o X||``; the loss, the feasibility gaps and the stopping rule are as without a mask.
+    Without penalties and ridge terms the observed error does not increase from one iteration to the next.  A mask
+    without a missing entry gives exactly the unmasked run.  The SVD and ALS starts need complete data and are refused
+    with a mask.  Data passed as ``PackedMatrices`` is filled in place during the fit and restored bit for bit on exit.
     """
     import torch
 
     from ._engine import PackedMatrices
 
     _check_svd_name(svd)
+    if mask is not None:
+        if isinstance(init, str) and (init in ("svd", "threshold_svd") or init in _ALS_INITS):
+            raise ValueError(f'init="{init}" needs complete data and cannot be combined with a mask; use init="random" '
+                             "or pass a factorization")
+        if not isinstance(matrices, PackedMatrices):
+            from ._engine import pack_mask
+
+            matrices = list(matrices)
+            mask = pack_mask(mask, [m.shape for m in matrices], require_observed=shard is None)
     if not torch.cuda.is_available():
         raise RuntimeError("matcouply_b200 needs a CUDA device (B200, sm_100a); there is no CPU fallback")
     if device is not None:
@@ -479,20 +507,36 @@ def cmf_aoadmm(
     # every kernel launch, workspace allocation and stream / event of the fit binds to `device`, whatever the caller's
     # current device is (the C ABI launches on torch's current stream, which belongs to the current device)
     with torch.cuda.device(device):
-        return _cmf_aoadmm_on_device(
-            matrices=matrices, rank=rank, init=init, n_iter_max=n_iter_max, l2_penalty=l2_penalty,
-            tv_penalty=tv_penalty, l1_penalty=l1_penalty, non_negative=non_negative, unimodal=unimodal,
-            generalized_l2_penalty=generalized_l2_penalty, l2_norm_bound=l2_norm_bound,
-            lower_bound=lower_bound, upper_bound=upper_bound, parafac2=parafac2, regs=regs,
-            feasibility_penalty_scale=feasibility_penalty_scale,
-            constant_feasibility_penalty=constant_feasibility_penalty, aux_init=aux_init,
-            dual_init=dual_init, svd=svd, init_params=init_params, random_state=random_state, tol=tol,
-            absolute_tol=absolute_tol, feasibility_tol=feasibility_tol, inner_tol=inner_tol,
-            inner_n_iter_max=inner_n_iter_max, update_A=update_A, update_B_is=update_B_is,
-            update_C=update_C, return_admm_vars=return_admm_vars, return_errors=return_errors,
-            verbose=verbose, process_group=process_group, shard=shard, gather_factors=gather_factors,
-            use_cuda_graph=use_cuda_graph, device=device,
-        )
+        saved = None
+        if mask is not None and isinstance(matrices, PackedMatrices):
+            # the caller's buffer is filled in place: keep its values at the missing positions and put them back on exit
+            from ._engine import MaskCSR, pack_mask, pack_mask_device
+
+            if isinstance(mask, torch.Tensor):
+                mask = pack_mask_device(mask, matrices, require_observed=shard is None)
+            elif not isinstance(mask, MaskCSR):
+                mask = pack_mask(mask, matrices.shapes, require_observed=shard is None)
+            mask = mask.to(device)
+            flat = mask.flat_index(matrices.X.shape[1])
+            saved = matrices.X.view(-1)[flat]
+        try:
+            return _cmf_aoadmm_on_device(
+                matrices=matrices, rank=rank, init=init, n_iter_max=n_iter_max, l2_penalty=l2_penalty,
+                tv_penalty=tv_penalty, l1_penalty=l1_penalty, non_negative=non_negative, unimodal=unimodal,
+                generalized_l2_penalty=generalized_l2_penalty, l2_norm_bound=l2_norm_bound,
+                lower_bound=lower_bound, upper_bound=upper_bound, parafac2=parafac2, regs=regs,
+                feasibility_penalty_scale=feasibility_penalty_scale,
+                constant_feasibility_penalty=constant_feasibility_penalty, aux_init=aux_init,
+                dual_init=dual_init, svd=svd, init_params=init_params, random_state=random_state, tol=tol,
+                absolute_tol=absolute_tol, feasibility_tol=feasibility_tol, inner_tol=inner_tol,
+                inner_n_iter_max=inner_n_iter_max, update_A=update_A, update_B_is=update_B_is,
+                update_C=update_C, return_admm_vars=return_admm_vars, return_errors=return_errors,
+                verbose=verbose, process_group=process_group, shard=shard, gather_factors=gather_factors,
+                use_cuda_graph=use_cuda_graph, device=device, mask=mask,
+            )
+        finally:
+            if saved is not None:
+                matrices.X.view(-1)[flat] = saved
 
 
 def _cmf_aoadmm_on_device(
@@ -534,8 +578,9 @@ def _cmf_aoadmm_on_device(
     shard=None,
     gather_factors=True,
     use_cuda_graph=None,
+    mask=None,
 ):
-    """Body of :func:`cmf_aoadmm`; runs with ``device`` as the current CUDA device."""
+    """Body of :func:`cmf_aoadmm`; runs with ``device`` as the current CUDA device.  ``mask``: None or a MaskCSR."""
     import torch
 
     from ._engine import AOADMMEngine, PackedMatrices
@@ -564,6 +609,14 @@ def _cmf_aoadmm_on_device(
                 int(s[0]) != int(j) for s, j in zip(packed.shapes, shard.row_counts[shard.lo:shard.hi])):
             raise ValueError("`matrices` must hold exactly the slices [shard.lo, shard.hi) of the global problem")
         shape_view = [_ShapeOnly((j, packed.K)) for j in shard.row_counts]  # the GLOBAL problem
+    if mask is not None:
+        counts = torch.tensor([mask.n_missing, mask.n_observed], dtype=torch.float64, device=device)
+        if process_group is not None:
+            torch.distributed.all_reduce(counts, group=process_group)
+        n_missing, n_observed = (int(v) for v in counts.tolist())
+        if n_observed == 0:
+            raise ValueError("the mask has no observed entry")
+        mask = mask.to(device) if n_missing else None  # no hole anywhere: exactly the unmasked run
     # default path: the big B-mode blocks (B_i, aux, dual) are drawn on the device from random_state's own MT19937
     # stream (bit-identical to host draws, see csrc/rng.cu); B2_HOST_RNG=1 forces the host draws
     dev_draw = None if os.environ.get("B2_HOST_RNG") else device
@@ -628,7 +681,8 @@ def _cmf_aoadmm_on_device(
                           feasibility_penalty_scale=feasibility_penalty_scale, constant_A=constant_A,
                           constant_B=constant_B, inner_n_iter_max=inner_n_iter_max,
                           update=(update_A, update_B_is, update_C), group=process_group,
-                          shard_rows=None if shard is None else (shard.lo, shard.n_global), inner_tol=inner_tol)
+                          shard_rows=None if shard is None else (shard.lo, shard.n_global), inner_tol=inner_tol,
+                          mask=mask)
     if shard is not None:
         from .distributed import shard_state
 
@@ -789,6 +843,7 @@ def parafac2_aoadmm(
     return_errors=False,
     return_admm_vars=False,
     verbose=False,
+    mask=None,
     **extra,
 ):
     """Alias of :func:`cmf_aoadmm` with the PARAFAC2 constraint on mode 1 (decomposition.py:1103-1179)."""
@@ -801,5 +856,5 @@ def parafac2_aoadmm(
         init_params=init_params, random_state=random_state, tol=tol, absolute_tol=absolute_tol,
         feasibility_tol=feasibility_tol, inner_tol=inner_tol, inner_n_iter_max=inner_n_iter_max, update_A=update_A,
         update_B_is=update_B_is, update_C=update_C, return_errors=return_errors, return_admm_vars=return_admm_vars,
-        verbose=verbose, **extra,
+        verbose=verbose, mask=mask, **extra,
     )
