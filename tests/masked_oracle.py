@@ -1,5 +1,5 @@
 """NumPy fp64 restatement of masked fitting (EM with one refill per outer iteration), the yardstick of
-tests/test_masked_cpu.py and tests/test_gpu_masked.py.
+tests/test_masked_cpu.py, tests/test_gpu_masked.py and tests/test_gpu_masked_width.py.
 
 It drives the oracle's own mode solvers, penalties and diagnostics (oracle/aoadmm_oracle.py, unchanged) with the
 masked semantics of ``cmf_aoadmm(..., mask=...)``:
@@ -28,6 +28,44 @@ def masked_fill(X_obs, obs, A, Bs, C):
 def observed_error(X_obs, obs, A, Bs, C):
     """‖M∘(X − X̂)‖, evaluated densely."""
     return np.sqrt(sum(np.sum(np.where(M, X - Xh, 0.0) ** 2) for X, M, Xh in zip(X_obs, obs, _model(A, Bs, C))))
+
+
+def refill_reference(x_old, row_ptr, col, gor, A, B, C, Y=None, dtype=np.float64, chunk=1 << 20):
+    """The contract of one ``b2_mask_refill`` launch (``_ops.mask_refill``) in float64, over the CSR list
+    ``(row_ptr, col)`` of the missing entries and their current values ``x_old`` (in CSR order):
+
+    - the missing entry (n, k) becomes x̂ = (B[n] ∘ A[gor[n]]) · C[k], rounded to ``dtype``; d = x̂ − x_old;
+    - Y[n] += Σ_k d·C[k] (rounded to ``dtype``);
+    - out[0] += Σ d², out[1] += Σ (x̂² − x_old²).
+
+    Returns dict(xhat = x̂ before the rounding, new = x̂ as stored, scale = |B∘A[gor]|·|C| per entry,
+    Y = the updated Y or None, yscale = |Y| + Σ_k |d|·|C[k]| per row, sums = (Σ d², Σ (x̂² − x_old²)),
+    sums_scale = Σ (x̂² + x_old²))."""
+    import scipy.sparse as sp
+
+    row_ptr, col = np.asarray(row_ptr, dtype=np.int64), np.asarray(col, dtype=np.int64)
+    N = len(row_ptr) - 1
+    rows = np.repeat(np.arange(N), np.diff(row_ptr))
+    W = np.asarray(B, dtype=np.float64) * np.asarray(A, dtype=np.float64)[np.asarray(gor)[:N]]
+    C = np.asarray(C, dtype=np.float64)
+    xhat, scale = np.empty(len(col)), np.empty(len(col))
+    for p in range(0, len(col), chunk):  # bounded temporaries at millions of entries
+        r, k = rows[p:p + chunk], col[p:p + chunk]
+        xhat[p:p + chunk] = np.einsum("er,er->e", W[r], C[k])
+        scale[p:p + chunk] = np.einsum("er,er->e", np.abs(W[r]), np.abs(C[k]))
+    new = xhat.astype(dtype).astype(np.float64)
+    x_old = np.asarray(x_old, dtype=np.float64)
+    d = new - x_old
+    res = dict(xhat=xhat, new=new, scale=scale, Y=None, yscale=None,
+               sums=(float(np.sum(d * d)), float(np.sum(new * new - x_old * x_old))),
+               sums_scale=float(np.sum(new * new + x_old * x_old)))
+    if Y is not None:
+        K = C.shape[0]
+        D = sp.csr_matrix((d, col, row_ptr), shape=(N, K))  # Σ_k d·C[k] per row as one sparse product
+        Y = np.asarray(Y, dtype=np.float64)
+        res["Y"] = (Y + D @ C).astype(dtype).astype(np.float64)
+        res["yscale"] = np.abs(Y) + abs(D) @ np.abs(C)
+    return res
 
 
 def ao_admm_masked(matrices, rank, mask, n_iter_max=1000, l2_penalty=None, l1_penalty=None, non_negative=None,

@@ -106,3 +106,42 @@ def test_mask_validation_messages():
             parafac2_aoadmm(X, 2, init=init, mask=[np.ones((4, 3)), np.ones((2, 3))])
     with pytest.raises(ValueError, match="complete data"):
         ao_admm_masked(X, 2, [np.ones((4, 3)), np.ones((2, 3))], init="svd")
+
+
+@pytest.mark.parametrize("dtype", [np.float64, np.float32])
+def test_refill_reference_agrees_with_the_oracle_semantics(dtype):
+    """The NumPy statement of one refill launch (``refill_reference``, the yardstick of the kernel tests) against the
+    dense formulas of the trajectory oracle: the refilled data is ``masked_fill``; ``‖F_old − X̂‖² − out[0]`` is the
+    ``observed_error`` squared (the engine's loss identity); ``out[1]`` is the change of ``‖F‖²``; and a ``Y = F_old C``
+    corrected by the refill is ``F_new C``.  Slices of 0 and 1 rows, a fully missing row and a complete row included."""
+    from masked_oracle import masked_fill, observed_error, refill_reference
+
+    rs = np.random.RandomState(5)
+    Js, K, R = [7, 0, 12, 1, 9], 37, 4
+    X, M = _ragged_problem(2, K=K, R=R, Js=Js, frac=0.3)
+    M[2][3], M[2][4] = False, True  # a fully missing row and a complete one
+    X = [x.astype(dtype).astype(np.float64) for x in X]
+    A, C = rs.uniform(size=(len(Js), R)), rs.standard_normal((K, R))
+    Bs = [rs.standard_normal((J, R)) for J in Js]
+    F_old = [np.where(m, x, rs.standard_normal(x.shape).astype(dtype)) for x, m in zip(X, M)]  # any previous fill
+    miss = ~np.concatenate(M, 0)
+    row_ptr = np.concatenate([[0], np.cumsum(miss.sum(axis=1))])
+    rows, col = np.nonzero(miss)
+    gor = np.repeat(np.arange(len(Js)), Js)
+    Fo, B = np.concatenate(F_old, 0), np.concatenate(Bs, 0)
+    Y_old = Fo @ C
+    ref = refill_reference(Fo[rows, col], row_ptr, col, gor, A, B, C, Y=Y_old, dtype=dtype)
+
+    Fn = Fo.copy()
+    Fn[rows, col] = ref["new"]
+    want = np.concatenate(masked_fill([np.where(m, x, 0.0) for x, m in zip(X, M)], M, A, Bs, C), 0)
+    tol = 1e-13 if dtype == np.float64 else 1e-6
+    np.testing.assert_allclose(Fn, want, rtol=tol, atol=tol)
+    np.testing.assert_array_equal(Fn[~miss], Fo[~miss])
+    Xh = np.concatenate([(b * A[i]) @ C.T for i, b in enumerate(Bs)], 0)
+    sse_obs = np.sum((Fo - Xh) ** 2) - ref["sums"][0]
+    # fp32: d is taken against the stored (rounded) x̂, as the kernel does
+    floor = 1e-12 if dtype == np.float64 else 1e-6
+    assert abs(sse_obs - observed_error(X, M, A, Bs, C) ** 2) <= floor * np.sum(Fo ** 2 + Xh ** 2)
+    assert abs(ref["sums"][1] - (np.sum(Fn ** 2) - np.sum(Fo ** 2))) <= 1e-13 * ref["sums_scale"]
+    assert np.all(np.abs(ref["Y"] - Fn @ C) <= (1e-12 if dtype == np.float64 else 1e-6) * (np.abs(Fn) @ np.abs(C)))
