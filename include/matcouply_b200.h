@@ -37,7 +37,9 @@ enum { B2_PEN_NONNEG = 0, B2_PEN_BOX = 1, B2_PEN_L1 = 2, B2_PEN_L2BALL = 3, B2_P
        /* column-coupled kinds finished by their own b2_prox_* call (penalties.py:595, :928, :750) */
        B2_PEN_GL2 = 6, B2_PEN_SIMPLEX = 7, B2_PEN_TV = 8,
        /* prox evaluated by the caller (user-defined ADMMPenalty subclass): the kernels only leave V = x + dual in `dual` */
-       B2_PEN_HOST = 9 };
+       B2_PEN_HOST = 9,
+       /* TemporalSmoothnessPenalty (mode 1 only): couples B_i to B_{i-1}; finished by b2_prox_temporal */
+       B2_PEN_TEMPORAL = 10 };
 
 /* how a row of an ADMM state matrix finds its group (slice) */
 enum { B2_GROUP_SINGLE = 0 /* every row -> group 0 (C-mode) */,
@@ -286,6 +288,37 @@ int b2_quadform(const void* M, const void* x, int n_groups, int J, int R, double
  * phase 2: pd = P Delta, dual = V - pd. */
 int b2_pf2_fixed_basis(void* pd, void* dual, const void* P, const void* Delta, const int64_t* row_off, int n_groups,
                        long long n, int R, const void* rho, double* num_part, int phase, int dtype, void* stream);
+
+/* ---- TemporalSmoothnessPenalty: lam * sum_{i>=1} ||B_i - B_{i-1}||_F^2 over the slice order (DESIGN.md §11) -------
+ * n_slices slices of equal height, packed one after the other: element (i, p) at i * n_pos + p with n_pos = J * R.
+ * For every position p:  (diag(rho) + 2 lam L) z = rho o v,  L the path-graph Laplacian of the slices; V arrives in
+ * `dual`, the call leaves aux = z and dual = V - aux (as stored).  rho: device array in the data's dtype,
+ * rho[i * rho_stride] (stride 0 = one value for all slices).  fp32 data is solved in fp64.  Partition solve in
+ * chunks of 32 slices; bit-reproducible (fixed order, no atomics).  ws: >= b2_prox_temporal_workspace_bytes(n_slices,
+ * n_pos, world) bytes, 8-byte aligned; its content must survive from stage 1 to stage 2.
+ * stage 0: the whole system (single GPU; world = 1, has_left = has_right = 0, xch may be NULL).
+ * Sharded runs (slices [lo, lo + n_slices) of a larger problem on this rank; has_left / has_right: the problem has
+ * slices before / after them):
+ *   stage 1: solve the local block with zero outer boundaries and write row `rank` of xch (world x (2 n_pos + 4)
+ *            doubles, zero-filled by the caller): [first-slice values (n_pos), last-slice values (n_pos), the first /
+ *            last entries of T_loc^-1 (2 lam e_first), of T_loc^-1 (2 lam e_last)]; aux / dual untouched.
+ *   (caller: sum-all-reduce xch over the ranks; ranks without slices contribute a zero row)
+ *   stage 2: solve the 2 x world reduced system (identically on every rank) and finish aux / dual. */
+int b2_prox_temporal(void* aux, void* dual, long long n_slices, long long n_pos, const void* rho, int rho_stride,
+                     double lam, int stage, int has_left, int has_right, double* xch, int world, int rank, int dtype,
+                     void* ws, size_t ws_bytes, void* stream);
+size_t b2_prox_temporal_workspace_bytes(long long n_slices, long long n_pos, int world);
+/* The same solve with one thread per position running Thomas over all n_slices slices (the forward sweep is parked
+ * in aux, in the data's dtype): the latency-bound baseline the partition solve is measured and tested against.
+ * ws as for stage 0 of b2_prox_temporal. */
+int b2_prox_temporal_serial(void* aux, void* dual, long long n_slices, long long n_pos, const void* rho,
+                            int rho_stride, double lam, int dtype, void* ws, size_t ws_bytes, void* stream);
+/* out[0] = lam * sum_i ||x_i - x_{i-1}||^2 over the local pairs; part: n_slices doubles of scratch (per-pair partials,
+ * summed in a fixed order).  Sharded: xch = world x (n_pos + 1) doubles, all-reduced, row r = [last slice of rank r,
+ * 1 if rank r holds slices]; the pair (last slice of the nearest earlier rank with slices, x_0) is added, so that
+ * every pair is counted on exactly one rank.  xch NULL: no such pair. */
+int b2_temporal_norm(const void* x, long long n_slices, long long n_pos, double lam, const double* xch, int rank,
+                     double* out, double* part, int dtype, void* stream);
 
 /* ---- masked fitting (missing entries, EM refill after every outer iteration; DESIGN.md §10) --------------------
  * Missing-entry refill.  For every packed row n (slice g = group_of_row[n]) and every missing column k in

@@ -29,7 +29,7 @@ from . import _lib, _ops
 
 
 # column-coupled kinds whose prox / penalty value is launched by the penalty object itself (penalties._EnginePenaltyMixin)
-_ENGINE_PROX_KINDS = (_lib.PEN_GL2, _lib.PEN_SIMPLEX, _lib.PEN_TV)
+_ENGINE_PROX_KINDS = (_lib.PEN_GL2, _lib.PEN_SIMPLEX, _lib.PEN_TV, _lib.PEN_TEMPORAL)
 
 # Kernel-fusion switches (tests flip them to cross-check the fused kernels against the one-kernel-per-step path).
 # "x1": the single-read fused X-stream pass for slice-local B-updates (csrc/xfused.cu): one pass over X per outer
@@ -367,6 +367,13 @@ class AOADMMEngine:
             if len(st.regs) > _lib.MAX_PENALTIES_PER_MODE:
                 raise ValueError(f"at most {_lib.MAX_PENALTIES_PER_MODE} penalties per mode are supported")
             st.desc = [r._descriptor() for r in st.regs]
+            if m != 1 and any(d[0] == _lib.PEN_TEMPORAL for d in st.desc):
+                raise ValueError(
+                    "TemporalSmoothnessPenalty can only be imposed with mode=1 (it couples B_i to B_(i-1)); for "
+                    f"smoothness over the rows of {'A' if m == 0 else 'C'} use GeneralizedL2Penalty with a path-graph "
+                    "Laplacian")
+        if any(d[0] == _lib.PEN_TEMPORAL for d in self.modes[1].desc):
+            self.temporal_height = self._common_slice_height(packed)
         for reg, (kind, *_) in zip(self.modes[0].regs, self.modes[0].desc):
             # a user-defined RowVectorPenalty has a row update; every other bridged / matrix-wise penalty needs ONE rho
             matrixwise = kind in _ENGINE_PROX_KINDS or (
@@ -473,6 +480,23 @@ class AOADMMEngine:
             self._ev_fork, self._ev_join = torch.cuda.Event(), torch.cuda.Event()
         self.n_xstream_launches = 0
         self.xstream_events = None  # set to {"y": [], "z": []} to record (start, end) CUDA events per launch
+
+    def _common_slice_height(self, packed):
+        """The height J shared by every slice of the (global) problem, for TemporalSmoothnessPenalty; sharded runs
+        reduce the local minimum and maximum, so that every rank takes the same decision (a rank without slices
+        learns J here)."""
+        heights = sorted(set(int(h) for h in np.diff(packed.row_offsets)))
+        if self.world > 1:
+            mm = torch.tensor([heights[-1] if heights else -1, -heights[0] if heights else -(2 ** 52)],
+                              dtype=torch.float64, device=self.dev)
+            self._allreduce(mm, "max")
+            lo_hi = (int(-mm[1].item()), int(mm[0].item()))
+            heights = sorted(set(lo_hi)) if lo_hi[1] >= 0 else []
+        if len(heights) > 1:
+            raise ValueError(
+                "TemporalSmoothnessPenalty needs factor matrices with the same number of rows (B_i - B_(i-1) is "
+                f"undefined otherwise); found heights {heights if self.world == 1 else 'from %d to %d' % lo_hi}")
+        return heights[0] if heights else 0
 
     # ------------------------------------------------------------------------------------------------------
     # state upload / download (host NumPy float64 <-> device)

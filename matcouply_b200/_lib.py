@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("B2_LIB_PATH_DEBUG") or os.path.join(_HERE, "libmatcou
 F32, F64 = 0, 1
 VARIANT_AUTO, VARIANT_FMA, VARIANT_DMMA = 0, 1, 2
 PEN_NONNEG, PEN_BOX, PEN_L1, PEN_L2BALL, PEN_UNIMODAL, PEN_PARAFAC2, PEN_GL2, PEN_SIMPLEX, PEN_TV, PEN_HOST = range(10)
+PEN_TEMPORAL = 10
 GROUP_SINGLE, GROUP_INDEXED, GROUP_IDENTITY = 0, 1, 2
 OPT_PF2_ROWPASS_MMA, OPT_POLAR_WARP, OPT_ADMM_LOCAL_MMA, OPT_XSTREAM_HYBRID, OPT_UNIMODAL_VARIANT = 0, 1, 2, 3, 4
 # B2_OPT_PF2_ROWPASS_MMA: 0 = shuffle kernel, 1 = DMMA tile kernel, 2 (default) = + the steady-state specialisation
@@ -80,6 +81,9 @@ _SIGNATURES = {
     "b2_mt19937_jump_host": [_vp, ctypes.c_ulonglong],
     "b2_set_option": [_i, _i],
     "b2_mask_refill": [_vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _i, _vp, _vp, _i, _vp, _sz, _vp],
+    "b2_prox_temporal": [_vp, _vp, _ll, _ll, _vp, _i, _d, _i, _i, _i, _vp, _i, _i, _i, _vp, _sz, _vp],
+    "b2_prox_temporal_serial": [_vp, _vp, _ll, _ll, _vp, _i, _d, _i, _vp, _sz, _vp],
+    "b2_temporal_norm": [_vp, _ll, _ll, _d, _vp, _i, _vp, _vp, _i, _vp],
 }
 _OTHER = {
     "b2_last_error": ([], ctypes.c_char_p),
@@ -94,6 +98,7 @@ _OTHER = {
     "b2_xstream_z_ldw": ([_i, _i, _i], _i),
     "b2_unimodal_workspace_bytes": ([_i, _i, _i], _sz),
     "b2_mask_refill_workspace_bytes": ([_ll], _sz),
+    "b2_prox_temporal_workspace_bytes": ([_ll, _ll, _i], _sz),
 }
 EXPORTED_SYMBOLS = sorted(list(_SIGNATURES) + list(_OTHER))
 

@@ -230,6 +230,32 @@ def tv_norm(x, row_off, n_groups, R, out):
     call("b2_tv_norm", _ptr(x), _ptr(row_off), n_groups, R, _ptr(out), _ptr(part), dtype_code(x.dtype), _stream())
 
 
+def prox_temporal_workspace(n_slices, n_pos, world, device):
+    """Scratch of b2_prox_temporal / b2_prox_temporal_serial for n_slices slices of n_pos = J * R entries."""
+    need = int(_lib.load().b2_prox_temporal_workspace_bytes(int(n_slices), int(n_pos), int(world)))
+    return torch.empty(max(need, 8), dtype=torch.uint8, device=device)
+
+
+def prox_temporal(aux, dual, n_slices, n_pos, rho, lam, ws, stage=0, has_left=False, has_right=False, xch=None,
+                  world=1, rank=0):
+    """rho: device tensor with one value per slice, or a single value shared by all slices.  Stage 0 solves the whole
+    system; stages 1 / 2 are the two halves of a sharded solve around the all-reduce of `xch` (see the C header)."""
+    call("b2_prox_temporal", _ptr(aux), _ptr(dual), int(n_slices), int(n_pos), _ptr(rho), 1 if rho.numel() > 1 else 0,
+         float(lam), int(stage), int(bool(has_left)), int(bool(has_right)), _ptr(xch), int(world), int(rank),
+         dtype_code(aux.dtype), _ptr(ws), ws.numel(), _stream())
+
+
+def prox_temporal_serial(aux, dual, n_slices, n_pos, rho, lam, ws):
+    call("b2_prox_temporal_serial", _ptr(aux), _ptr(dual), int(n_slices), int(n_pos), _ptr(rho),
+         1 if rho.numel() > 1 else 0, float(lam), dtype_code(aux.dtype), _ptr(ws), ws.numel(), _stream())
+
+
+def temporal_norm(x, n_slices, n_pos, lam, out, part, xch=None, rank=0):
+    """out[0] = lam * sum_i ||x_i - x_{i-1}||^2; part: >= n_slices doubles of scratch."""
+    call("b2_temporal_norm", _ptr(x), int(n_slices), int(n_pos), float(lam), _ptr(xch), int(rank), _ptr(out),
+         _ptr(part), dtype_code(x.dtype), _stream())
+
+
 def prox_gl2(aux, dual, n_groups, J, R, U, s, rho, tmp):
     call("b2_prox_gl2", _ptr(aux), _ptr(dual), n_groups, J, R, _ptr(U), _ptr(s), _ptr(rho),
          1 if rho.numel() > 1 else 0, _ptr(tmp), dtype_code(aux.dtype), _stream())

@@ -125,7 +125,7 @@ inline int b2_pack_penalties(const b2_penalty_desc* pens, int n_pen, PenArgs* pa
     B2_REQUIRE(n_pen >= 0 && n_pen <= kMaxPen, "at most %d penalties per mode are supported (got %d)", kMaxPen, n_pen);
     pa->n_pen = n_pen;
     for (int p = 0; p < n_pen; ++p) {
-        B2_REQUIRE(pens[p].kind >= B2_PEN_NONNEG && pens[p].kind <= B2_PEN_HOST, "unknown penalty kind %d",
+        B2_REQUIRE(pens[p].kind >= B2_PEN_NONNEG && pens[p].kind <= B2_PEN_TEMPORAL, "unknown penalty kind %d",
                    pens[p].kind);
         B2_REQUIRE(pens[p].aux && pens[p].dual, "penalty %d: aux/dual pointers must be set", p);
         pa->kind[p] = pens[p].kind;

@@ -9,7 +9,8 @@ methods (``factor_matrix_update`` ...) are also callable on their own with NumPy
 run the same CUDA kernels through the C ABI and return the input's array type.  There is no CPU implementation.
 
 ``GeneralizedL2Penalty`` (:595), ``TotalVariationPenalty`` (:750) and ``UnitSimplex`` (:928) run their proximal
-operators as CUDA kernels too (csrc/prox_extra.cu); user-defined subclasses that implement the protocol in Python are
+operators as CUDA kernels too (csrc/prox_extra.cu), as does ``TemporalSmoothnessPenalty`` (no reference counterpart:
+smoothness of the ``B_i`` over the slice order, csrc/prox_temporal.cu); user-defined subclasses that implement the protocol in Python are
 bridged by the engine (``PEN_HOST``: the pre-image is handed to the Python method, the result goes back to HBM).
 """
 from abc import ABC, abstractmethod
@@ -21,7 +22,7 @@ from . import _lib
 __all__ = [
     "ADMMPenalty", "MatricesPenalty", "MatrixPenalty", "RowVectorPenalty", "HardConstraintMixin", "NonNegativity",
     "Box", "L1Penalty", "L2Ball", "Unimodality", "Parafac2", "GeneralizedL2Penalty", "TotalVariationPenalty",
-    "UnitSimplex",
+    "UnitSimplex", "TemporalSmoothnessPenalty",
 ]
 
 
@@ -711,3 +712,138 @@ class UnitSimplex(_EnginePenaltyMixin, HardConstraintMixin, MatrixPenalty):
 
     def penalty(self, x):
         return 0
+
+
+class TemporalSmoothnessPenalty(_EnginePenaltyMixin, MatricesPenalty):
+    """Smoothness of the mode-1 factor matrices over the slice order (temporal PARAFAC2 / CMF):
+
+        g(B_0, ..., B_{I-1}) = smoothness_reg * sum_{i=1}^{I-1} ||B_i - B_{i-1}||_F^2
+
+    i.e. ``x^T (smoothness_reg L) x`` with ``L`` the path-graph Laplacian over the slices, for every entry (j, r), in
+    the convention of ``GeneralizedL2Penalty``.  The prox ``argmin g(Z) + sum_i rho_i / 2 ||Z_i - V_i||^2`` solves the
+    tridiagonal system ``(diag(rho) + 2 smoothness_reg L) z = rho o v`` for every entry; all slices must have the same
+    number of rows.  Mode 1 only (for smoothness over the rows of ``A`` or ``C`` use ``GeneralizedL2Penalty`` with a
+    path-graph Laplacian).  The solve is a partition (spike) solve on the device (csrc/prox_temporal.cu); in a sharded
+    run every rank is one block of it and the ranks exchange one small buffer per call."""
+
+    _kind = _lib.PEN_TEMPORAL
+
+    def __init__(self, smoothness_reg, aux_init="random_uniform", dual_init="random_uniform"):
+        if not smoothness_reg > 0:
+            raise ValueError("The smoothness regularization strength must be positive.")
+        super().__init__(aux_init, dual_init)
+        self.smoothness_reg = smoothness_reg
+        self._ws = {}  # (n_slices, n_pos, world, device) -> device workspace of b2_prox_temporal
+
+    def _descriptor(self):
+        return (_lib.PEN_TEMPORAL, False, float(self.smoothness_reg), 0.0)
+
+    @staticmethod
+    def _check_heights(heights):
+        found = sorted(set(int(h) for h in heights))
+        if len(found) > 1:
+            raise ValueError(
+                "TemporalSmoothnessPenalty needs factor matrices with the same number of rows (B_i - B_(i-1) is "
+                f"undefined otherwise); found heights {found}")
+        return found[0] if found else 0
+
+    def _workspace(self, n_slices, n_pos, world, device):
+        from . import _ops
+
+        key = (int(n_slices), int(n_pos), int(world), str(device))
+        if key not in self._ws:
+            self._ws[key] = _ops.prox_temporal_workspace(n_slices, n_pos, world, device)
+        return self._ws[key]
+
+    def _shape(self, eng, x, n_groups, max_rows, n_rows):
+        """(slice height J, entries per slice J * R).  In an engine the height is the one checked at set-up, which
+        a rank without slices also knows (the exchange buffers of a sharded run must have the same size on every
+        rank)."""
+        if eng is not None:
+            J = eng.temporal_height
+        else:
+            J = int(max_rows) if n_groups else 0
+            if n_groups * J != n_rows:
+                raise ValueError(f"TemporalSmoothnessPenalty needs slices of equal height ({n_rows} rows in {n_groups} "
+                                 f"slices of at most {max_rows} rows)")
+        return J, J * x.shape[1]
+
+    def _engine_prox(self, eng, aux, dual, row_off, n_groups, max_rows, rho, n_rows):
+        import torch
+
+        from . import _ops
+
+        I = int(n_groups)
+        _, P = self._shape(eng, aux, n_groups, max_rows, n_rows)
+        lam = float(self.smoothness_reg)
+        world = 1 if eng is None else eng.world
+        ws = self._workspace(I, P, world, aux.device)
+        if world == 1:
+            _ops.prox_temporal(aux, dual, I, P, rho, lam, ws)
+            return
+        # sharded: this rank's slices are one block of the partition solve; the local solution's end values and the
+        # ends of its two spike vectors go through one all-reduce, then every rank solves the 2 x world system
+        lo, I_glob = eng.shard_rows
+        rank = torch.distributed.get_rank(eng.group)
+        xch = torch.zeros((world, 2 * P + 4), dtype=torch.float64, device=aux.device)
+        kw = dict(has_left=lo > 0, has_right=lo + I < I_glob, xch=xch, world=world, rank=rank)
+        _ops.prox_temporal(aux, dual, I, P, rho, lam, ws, stage=1, **kw)
+        eng._allreduce(xch)
+        _ops.prox_temporal(aux, dual, I, P, rho, lam, ws, stage=2, **kw)
+
+    def _engine_penalty(self, eng, x, row_off, n_groups, max_rows, n_rows, out):
+        import torch
+
+        from . import _ops
+
+        I = int(n_groups)
+        J, P = self._shape(eng, x, n_groups, max_rows, n_rows)
+        part = torch.empty(max(I, 1), dtype=torch.float64, device=x.device)
+        lam = float(self.smoothness_reg)
+        if eng is None or eng.world == 1:
+            _ops.temporal_norm(x, I, P, lam, out, part)
+            return
+        # sharded: the pair (last slice of the previous rank with slices, first local slice) is counted here
+        rank = torch.distributed.get_rank(eng.group)
+        xch = torch.zeros((eng.world, P + 1), dtype=torch.float64, device=x.device)
+        if I > 0:
+            xch[rank, :P] = x[(I - 1) * J:].reshape(-1)
+            xch[rank, P] = 1.0
+        eng._allreduce(xch)
+        _ops.temporal_norm(x, I, P, lam, out, part, xch=xch, rank=rank)
+
+    def factor_matrices_update(self, factor_matrices, feasibility_penalties, auxes):
+        import torch
+
+        from . import _ops
+
+        devs = [_Dev(fm) for fm in factor_matrices]
+        if not devs:
+            return []
+        self._check_heights(d.t.shape[0] for d in devs)
+        dtype = devs[0].t.dtype
+        V = torch.cat([d.t.to(dtype).reshape(-1) for d in devs]).contiguous()
+        I, P = len(devs), V.numel() // len(devs)
+        rho = torch.as_tensor(np.asarray([float(r) for r in feasibility_penalties]), dtype=dtype).cuda()
+        aux = torch.empty_like(V)
+        _ops.prox_temporal(aux, V, I, P, rho, float(self.smoothness_reg), self._workspace(I, P, 1, V.device))
+        return [d.back(a.view(d.t.shape)) for d, a in zip(devs, aux.view(I, P))]
+
+    def penalty(self, x):
+        import torch
+
+        from . import _ops
+
+        if not isinstance(x, list):
+            raise TypeError("Cannot compute the temporal smoothness penalty of other types than a list of tensors")
+        devs = [_Dev(xi) for xi in x]
+        if len(devs) < 2:
+            return 0.0
+        self._check_heights(d.t.shape[0] for d in devs)
+        dtype = devs[0].t.dtype
+        X = torch.cat([d.t.to(dtype).reshape(-1) for d in devs]).contiguous()
+        I = len(devs)
+        out = torch.zeros(1, dtype=torch.float64, device="cuda")
+        part = torch.empty(I, dtype=torch.float64, device="cuda")
+        _ops.temporal_norm(X, I, X.numel() // I, float(self.smoothness_reg), out, part)
+        return float(out.item())
